@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Planner-step benchmark (contract: one JSON line on rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode train|fwd]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode train|fwd] [--dump-outputs DIR]
 
 Metric (BASELINE.json): planner steps/s at B=64 episodes per GPU, 12 views, 80-node graph, 200-token
 instruction, 6 cross-modal layers (BASELINE.json configs[2]; the reference checkpoints use 4 — pass
@@ -32,6 +32,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 from etpnav_b200.config import PlannerConfig            # noqa: E402
 from etpnav_b200.synth import make_inputs, make_weights, step_flops  # noqa: E402
@@ -92,7 +93,14 @@ def parse():
     ap.add_argument("--workload", default="planner", choices=["planner", "pretrain", "packing"],
                     help="planner (default, BASELINE.json's metric) | pretrain (SURVEY.md 8f N2: one pre-training iteration "
                          "of the twin, mlm and sap alternating) | packing (8f N3: the per-step map / view packing)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="planner workload: after the timed steps write what the last timed step computed as DIR/<name>.npy "
+                         "(float32; the inputs are seeded, so two builds can be compared output for output)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.workload != "planner" or a.impl != "b200"):
+        ap.error("--dump-outputs covers the planner workload of the b200 arm")
     pre = PRESETS[a.config]
     for k in ("batch", "views", "nodes", "tokens", "x_layers", "text_law"):
         if getattr(a, k) is None:
@@ -540,6 +548,34 @@ def run_packing_workload(a):
 # ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
+# per array (16 MiB of float32).  At most four arrays are written and two of them (masks, logits) are small, so a dump
+# stays under 64 MB.
+DUMP_MAX_ELEMS = 1 << 22
+
+
+def dump_outputs(path, arrays, model=None):
+    """``--dump-outputs``: every array the last timed step handed its caller and, after a training step, the parameters it
+    updated in place (all of them in name order), as float32 DIR/<name>.npy.  An array larger than DUMP_MAX_ELEMS is
+    replaced by a fixed, seeded sample of its flattened entries (the same indices for every build at the same shape).
+    The node logits are -inf at masked nodes (visited or padding): an array with -inf entries is written with 0 there,
+    and DIR/<name>_masked.npy holds 1 where they were, so every file is finite (NaN and +inf are left as they are)."""
+    import numpy as np
+    arrays = dict(arrays)
+    if model is not None:
+        arrays["params"] = torch.cat([p.detach().flatten() for _, p in sorted(model.named_parameters())])
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.flatten()[idx.to(t.device)]
+        masked = t == float("-inf")
+        if bool(masked.any()):
+            np.save(os.path.join(path, name + "_masked.npy"), masked.float().cpu().numpy())
+            t = t.masked_fill(masked, 0.0)
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def _latest_profile(prefix_glob):
     import glob
     c = sorted(glob.glob(os.path.join(ROOT, "profiles", prefix_glob)))
@@ -553,6 +589,9 @@ def main():
     # processes, 178-183 in others, same box, the copy alone at 55 GB/s in both).  Must be set before the CUDA context exists.
     os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
     a = parse()
+    # train mode's dropout seed stream starts at torch.initial_seed() (plus the rank): fixed, so that two runs with the same
+    # arguments compute the same step (--dump-outputs)
+    torch.manual_seed(0)
     if a.workload == "pretrain":
         return run_pretrain_workload(a)
     if a.workload == "packing":
@@ -607,6 +646,7 @@ def main():
     h2d_bytes = int(blob_meta[2])
     logits_host = torch.empty(B, N, dtype=torch.float32).pin_memory()
     d2h_bytes = logits_host.numel() * 4
+    last = {}       # what the latest step handed its caller (--dump-outputs)
 
     if mode == "train":
         model.train()
@@ -617,7 +657,8 @@ def main():
         def step(d):
             # training-loop form of the step: the compute stream returns once the navigation buckets are updated, the
             # panorama buckets finish under the next step's first GEMM; every timed region ends with trainer.join()
-            return trainer.step(d, pipelined=True)
+            last["global_logits"] = trainer.step(d, pipelined=True)
+            return last["global_logits"]
 
         step_done = trainer.join
     else:
@@ -630,10 +671,11 @@ def main():
 
         def step(d):
             with torch.no_grad():
-                model.forward_panorama(*[d[k] for k in keys_pano])
+                last["pano_embeds"], last["pano_masks"] = model.forward_panorama(*[d[k] for k in keys_pano])
                 out = model.forward_navigation(text_kv if text_kv is not None else d["txt_embeds"], d["txt_masks"], None,
                                                d["gmap_step_ids"], d["gmap_img_fts"], d["gmap_pos_fts"], d["gmap_masks"],
                                                d["gmap_visited_masks"], d["gmap_pair_dists"])
+            last.update(out)
             return out["global_logits"]
 
     def barrier():
@@ -677,6 +719,8 @@ def main():
     clk.__enter__()   # sampled across the timed regions below (value, e2e): all under load
     total_ms = timed(lambda: step(resident), a.steps)
     launches = lib.etp_launch_count() - n0
+    if a.dump_outputs and rank == 0:     # before any later pass runs another step
+        dump_outputs(a.dump_outputs, last, model if mode == "train" else None)
     ms_per_step = total_ms / a.steps
     value = world / (ms_per_step * 1e-3)
 

@@ -1,13 +1,13 @@
-"""Generate tests/golden_grads/c1_bert.pt by running the UNMODIFIED reference (authoring container only).
+"""Generate tests/golden/grads/c1_bert.pt by running the UNMODIFIED reference (oracle/ref_import.py).
 
 TEST INFRASTRUCTURE.  Usage:  python -m oracle.make_golden_grads
 The c1_bert fixture of tests/golden stores a 10-number signature per parameter gradient.  A full copy of the 140 M
 gradients would be 563 MB, so this companion fixture stores, for every parameter of the pano / nav groups (the ones the
 planner step trains), a SKETCH of the reference's fp32 gradient that pins every region of the tensor:
   1-D tensors: the full gradient;
-  2-D tensors: all row sums, all column sums and two full rows (indices drawn from a fixed generator).
+  2-D tensors: all row sums, all column sums and 64 single entries (flat indices drawn from a fixed generator).
 A sign or indexing error confined to a slice of a weight gradient (one head, one k-block, one output tile) moves the
-row / column sums of that slice; tests/test_backward_gpu.py compares every vector.
+row / column sums of that slice; tests/test_backward_gpu.py compares every vector.  The sketch stays under 1 MB.
 """
 import os
 import sys
@@ -20,13 +20,14 @@ from etpnav_b200.synth import make_inputs, make_weights  # noqa: E402
 from oracle import ref_import                          # noqa: E402
 from oracle.make_golden import CASES                   # noqa: E402
 
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden_grads")
+OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "grads")
 TEXT_PREFIXES = ("lang_encoder", "embeddings.word", "embeddings.position", "embeddings.LayerNorm")
+SAMPLE = 64     # single entries per 2-D gradient
 
 
-def sketch_rows(shape, name):
+def sketch_entries(shape, name):
     g = torch.Generator().manual_seed(sum(map(ord, name)) + 123)
-    return torch.randint(0, shape[0], (2,), generator=g)
+    return torch.randint(0, shape[0] * shape[1], (SAMPLE,), generator=g)
 
 
 def sketch(name, grad):
@@ -34,8 +35,9 @@ def sketch(name, grad):
     if g.dim() < 2:
         return {"full": g.clone()}
     g2 = g.reshape(g.shape[0], -1)
-    rows = sketch_rows(g2.shape, name)
-    return {"row_sum": g2.double().sum(1).float(), "col_sum": g2.double().sum(0).float(), "rows": rows, "row_vals": g2[rows].clone()}
+    idx = sketch_entries(g2.shape, name)
+    return {"row_sum": g2.double().sum(1).float(), "col_sum": g2.double().sum(0).float(), "idx": idx,
+            "vals": g2.flatten()[idx].clone()}
 
 
 def run(name="c1_bert"):

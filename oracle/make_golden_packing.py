@@ -1,4 +1,4 @@
-"""Generate tests/golden_packing/*.pt by running the UNMODIFIED reference packing code (authoring container only).
+"""Generate tests/golden/packing/*.pt by running the UNMODIFIED reference packing code (oracle/ref_import.py).
 
 TEST INFRASTRUCTURE.  Usage:  python -m oracle.make_golden_packing
 Episodes are simulated on the reference's own ``GraphMap`` (vlnce_baselines/models/graph_utils.py:133, imported as is):
@@ -19,7 +19,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import packing_port as PK   # noqa: E402
 from oracle import ref_import           # noqa: E402
 
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden_packing")
+OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "packing")
 
 
 def yaw_quat(theta):

@@ -1,4 +1,4 @@
-"""Generate tests/golden_pretrain/*.pt by running the UNMODIFIED reference pre-training model (authoring container only).
+"""Generate tests/golden/pretrain/*.pt by running the UNMODIFIED reference pre-training model (oracle/ref_import.py).
 
 TEST INFRASTRUCTURE.  Usage:  python -m oracle.make_golden_pretrain
 Each fixture stores the case definition (config, shapes, seeds) and what ``GlocalTextPathCMTPreTraining``
@@ -17,7 +17,7 @@ from etpnav_b200.config import PlannerConfig              # noqa: E402
 from etpnav_b200.synth import make_traj_batch, make_weights  # noqa: E402
 from oracle import ref_import                              # noqa: E402
 
-OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden_pretrain")
+OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "pretrain")
 _PT = dict(use_lang2visn_attn=True, mlm_head=True)
 
 CASES = {

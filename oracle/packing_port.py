@@ -11,7 +11,7 @@ habitat-lab v0.1.7 (``habitat.utils.geometry_utils.quaternion_from_coeff / quate
 numpy-quaternion, both absent from /root/reference: their published algorithm (Hamilton product q v q^-1, coefficients
 ordered [x, y, z, w]; polar angle = arctan2(y, x)) is restated in ``heading_from_quaternion``.
 Pinned by ``oracle/make_golden_packing.py``, which runs the reference's own GraphMap and the two trainer methods (the
-function bodies are executed from the reference source, unmodified) -> ``tests/golden_packing/*.pt``.
+function bodies are executed from the reference source, unmodified) -> ``tests/golden/packing/*.pt``.
 """
 import numpy as np
 import torch

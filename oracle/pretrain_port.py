@@ -4,7 +4,7 @@ Restates ``GlocalTextPathCMT`` / ``GlocalTextPathCMTPreTraining`` (paths relativ
 /root/reference/pretrain_src/pretrain_src/model) in plain tensor algebra on the raw ``state_dict`` (keys in the planner
 namespace, i.e. without the ``bert.`` prefix), reusing ``oracle/planner_port.py`` for the layers both models share.
 Pinned by ``oracle/make_golden_pretrain.py`` (the UNMODIFIED reference run in the authoring container on seeded
-synthetic batches -> ``tests/golden_pretrain/*.pt``) and ``tests/test_oracle_pretrain.py``.
+synthetic batches -> ``tests/golden/pretrain/*.pt``) and ``tests/test_oracle_pretrain.py``.
 """
 import torch
 import torch.nn.functional as F

@@ -8,7 +8,7 @@ from etpnav_b200.config import PlannerConfig
 from etpnav_b200.synth import make_inputs, make_weights
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-GOLDEN_GRADS_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_grads")
+GOLDEN_GRADS_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "grads")
 
 # bf16-operand mode (GEMM / attention operands rounded to bf16, fp32 everywhere else) against the fp32 reference:
 # <= 2x the envelope measured on B200 (profiles/r01_parity_report_final.jsonl: logits 0.0037-0.0089, embeddings
@@ -42,9 +42,11 @@ def load_case(name):
     return gold, cfg, sd, inp
 
 
-def slim(gold, t):
-    s = gold["case"].get("slim")
-    return t[:, ::s] if (s and t.dim() == 3) else t
+def slim(gold, t, key=None):
+    """The rows of ``t`` the fixture stores under ``key`` (oracle/make_golden.py: the case's ``slim`` and ``stride``)."""
+    c = gold["case"]
+    s = (c.get("slim") or 1) * c.get("stride", {}).get(key, 1)
+    return t[:, ::s] if (s > 1 and t.dim() == 3) else t
 
 
 def grad_sig(t):

@@ -12,7 +12,7 @@ from etpnav_b200.config import PlannerConfig
 from etpnav_b200.synth import make_traj_batch, make_weights
 from oracle import pretrain_port as PP
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_pretrain")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pretrain")
 
 
 def names():

@@ -1,5 +1,5 @@
 """CPU: the packing oracle (oracle/packing_port.py) reproduces what the UNMODIFIED reference packing code produced
-(tests/golden_packing, oracle/make_golden_packing.py): ETPTrainer._nav_gmap_variable / _vp_feature_variable and
+(tests/golden/packing, oracle/make_golden_packing.py): ETPTrainer._nav_gmap_variable / _vp_feature_variable and
 GraphMap.get_pos_fts.  Bit-exact: the port follows the reference's numpy operation order."""
 import glob
 import os
@@ -10,7 +10,7 @@ import torch
 
 from oracle import packing_port as PK
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden_packing")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "packing")
 
 
 def load(name):

@@ -1,5 +1,5 @@
 """GPU: caller-side packing (etpnav_b200/packing.py, SURVEY.md §8f N3) through the C ABI against the fixtures produced
-by the UNMODIFIED reference packing code (tests/golden_packing): pack_gmap vs ETPTrainer._nav_gmap_variable,
+by the UNMODIFIED reference packing code (tests/golden/packing): pack_gmap vs ETPTrainer._nav_gmap_variable,
 pack_vp_features vs _vp_feature_variable.  Integer / bool tensors and all distances bit-exact; sin / cos within 1 ulp;
 image features to fp32 rounding of x * (1/count) vs x / count."""
 import numpy as np

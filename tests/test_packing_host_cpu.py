@@ -1,7 +1,7 @@
 """CPU: the product's host packer (etpnav_b200/packing.py: flatten_gmaps, heading_from_quaternion) and the geometry
 code the etp_gmap_pack kernel runs (etpnav_b200/csrc/gmap_pack.cuh, compiled here for the HOST by
 tests/host_harness/gmap_pack_host.cpp — test infrastructure, not shipped) against the fixtures the unmodified reference
-produced (tests/golden_packing).  Distances / step ids / masks bit-exact; sin / cos of the float32 angles within 1 ulp
+produced (tests/golden/packing).  Distances / step ids / masks bit-exact; sin / cos of the float32 angles within 1 ulp
 (libm sinf vs numpy's float32 sin)."""
 import ctypes as C
 import os

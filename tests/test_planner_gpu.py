@@ -55,11 +55,12 @@ def test_forward_matches_golden(name):
                                    d["gmap_pos_fts"], d["gmap_masks"], d["gmap_visited_masks"], d["gmap_pair_dists"])
     torch.cuda.synchronize()
     tm = inp["txt_masks"]
-    e_txt = (slim(gold, txt.cpu()) - gold["txt_embeds"]).abs()
-    e_txt_valid = e_txt[slim(gold, tm[..., None].expand_as(txt))[..., 0]] if not gold["case"].get("slim") else e_txt
+    e_txt = (slim(gold, txt.cpu(), "txt_embeds") - gold["txt_embeds"]).abs()
+    e_txt_valid = (e_txt[slim(gold, tm[..., None].expand_as(txt), "txt_embeds")[..., 0]] if not gold["case"].get("slim")
+                   else e_txt)
     assert torch.equal(pmask.cpu(), gold["pano_masks"])
-    e_pano = (slim(gold, pano.cpu()) - gold["pano_embeds"]).abs()
-    e_emb = (slim(gold, nav["gmap_embeds"].cpu()) - gold["gmap_embeds"]).abs()
+    e_pano = (slim(gold, pano.cpu(), "pano_embeds") - gold["pano_embeds"]).abs()
+    e_emb = (slim(gold, nav["gmap_embeds"].cpu(), "gmap_embeds") - gold["gmap_embeds"]).abs()
     lg, lr = nav["global_logits"].cpu(), gold["global_logits"]
     assert torch.equal(torch.isinf(lg), torch.isinf(lr)), "-inf pattern differs"
     fin = ~torch.isinf(lr)

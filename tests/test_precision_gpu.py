@@ -93,8 +93,9 @@ def test_high_precision_forward_in_northstar_band(name):
     fin = ~torch.isinf(lr)
     ok_log = _in_band(lg[fin], lr[fin])
     e_log = (lg[fin] - lr[fin]).abs()
-    checks = {"txt": (slim(gold, txt.cpu()), gold["txt_embeds"]), "pano": (slim(gold, pano.cpu()), gold["pano_embeds"]),
-              "gmap": (slim(gold, nav["gmap_embeds"].cpu()), gold["gmap_embeds"])}
+    checks = {"txt": (slim(gold, txt.cpu(), "txt_embeds"), gold["txt_embeds"]),
+              "pano": (slim(gold, pano.cpu(), "pano_embeds"), gold["pano_embeds"]),
+              "gmap": (slim(gold, nav["gmap_embeds"].cpu(), "gmap_embeds"), gold["gmap_embeds"])}
     rep = {"case": name, "mode": "high", "logit_max": e_log.max().item(), "frac_in_northstar_band": ok_log.float().mean().item()}
     for k, (x, r) in checks.items():
         rep[k + "_max"] = (x - r).abs().max().item()

@@ -1,5 +1,5 @@
 """GPU: the pre-training twin (etpnav_b200/pretrain.py: B200TextPathCMT / B200PreTraining, SURVEY.md §8f N2) through
-the C ABI against the fixtures minted from the UNMODIFIED reference pre-training model (tests/golden_pretrain,
+the C ABI against the fixtures minted from the UNMODIFIED reference pre-training model (tests/golden/pretrain,
 oracle/make_golden_pretrain.py) and against the fp32 oracle port's autograd.  Same numerical contract as the
 navigation model's tests (tests/test_planner_gpu.py, tests/test_backward_gpu.py): bf16 GEMM operands, fp32 everything
 else; bit-exact -inf pattern and node selection, absolute envelopes for the embeddings / logits, relative L2 for
