@@ -54,8 +54,9 @@ __global__ void __launch_bounds__(256) attn_bwd_dq_kernel(const AttnBwdArgs a, i
   const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kTile;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int Sk = a.Sk;
-  stage_rows(Ks, a.k + static_cast<size_t>(b) * Sk * a.ldk + h * kD, Sk, a.ldk);
-  stage_rows(Vs, a.v + static_cast<size_t>(b) * Sk * a.ldv + h * kD, Sk, a.ldv);
+  const int kvb = a.kv_rows ? __ldg(a.kv_rows + b) : b;  // row of the K / V tensor this batch element reads
+  stage_rows(Ks, a.k + static_cast<size_t>(kvb) * Sk * a.ldk + h * kD, Sk, a.ldk);
+  stage_rows(Vs, a.v + static_cast<size_t>(kvb) * Sk * a.ldv + h * kD, Sk, a.ldv);
   for (int j = threadIdx.x; j < sk_pad; j += 256) {
     float m = -INFINITY;
     if (j < Sk) m = (a.key_valid == nullptr || a.key_valid[static_cast<size_t>(b) * Sk + j]) ? 0.f : a.mask_value;
@@ -136,6 +137,7 @@ __global__ void __launch_bounds__(256) attn_bwd_dkv_kernel(const AttnBwdArgs a, 
   const int b = blockIdx.z, h = blockIdx.y, k0 = blockIdx.x * kTile;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int Sq = a.Sq, Sk = a.Sk;
+  const size_t kvb = a.kv_rows ? __ldg(a.kv_rows + b) : b;  // K / V are read from this row; dK / dV go to row b
   stage_rows(Qs, a.q + static_cast<size_t>(b) * Sq * a.ldq + h * kD, Sq, a.ldq);
   stage_rows(dOs, a.dout + static_cast<size_t>(b) * Sq * a.lddo + h * kD, Sq, a.lddo);
   for (int i = threadIdx.x; i < sq_pad; i += 256) {
@@ -154,8 +156,9 @@ __global__ void __launch_bounds__(256) attn_bwd_dkv_kernel(const AttnBwdArgs a, 
     const int j = k0 + ki;
     if (j >= Sk) break;
     const size_t krow = static_cast<size_t>(b) * Sk + j;
-    const float2 fk = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(a.k + krow * a.ldk + h * kD + lane * 2));
-    const float2 fv = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(a.v + krow * a.ldv + h * kD + lane * 2));
+    const size_t kvrow = kvb * Sk + j;
+    const float2 fk = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(a.k + kvrow * a.ldk + h * kD + lane * 2));
+    const float2 fv = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(a.v + kvrow * a.ldv + h * kD + lane * 2));
     myk[lane * 2] = fk.x * a.scale; myk[lane * 2 + 1] = fk.y * a.scale;
     myv[lane * 2] = fv.x; myv[lane * 2 + 1] = fv.y;
     const float kbias = (a.key_valid == nullptr || a.key_valid[krow]) ? 0.f : a.mask_value;
@@ -200,6 +203,7 @@ int attention_bwd(const AttnBwdArgs& a, cudaStream_t stream) {
   ETP_REQUIRE(a.q && a.k && a.v && a.out && a.dout && a.lse && a.dvec && a.dq && a.dk && a.dv, "attention_bwd: null argument");
   ETP_REQUIRE(a.ldq % 8 == 0 && a.ldk % 8 == 0 && a.ldv % 8 == 0 && a.lddo % 8 == 0 && a.ldo % 2 == 0 && a.lddq % 2 == 0 &&
                   a.lddk % 2 == 0 && a.lddv % 2 == 0, "attention_bwd: pitches");
+  ETP_REQUIRE(a.kv_rows == nullptr || a.kv_B > 0, "attention_bwd: kv_B must be given with kv_rows");
   const int sk_pad = (a.Sk + 31) / 32 * 32, sq_pad = (a.Sq + 31) / 32 * 32;
   const size_t smem_a = static_cast<size_t>(sk_pad) * kStr * 2 * 2 + 2 * 8 * kD * 4 + 8 * static_cast<size_t>(sk_pad) * 4 +
                         static_cast<size_t>(sk_pad) * 4;

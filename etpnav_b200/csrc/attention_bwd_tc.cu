@@ -53,6 +53,7 @@ struct BwdDev {
   int lddq, lddk, lddv;
   float *dpair_w, *dpair_b;
   Drop drop;  // the forward's attention-probability dropout (thr 0 = off)
+  const int32_t* kv_rows;  // optional batch-row map of the K / V tensor (see AttnBwdArgs)
   unsigned long long* dbg;  // optional timeline of CTA 0 (globaltimer ns): [0,64) control thread, [64,128) math thread 0
 };
 
@@ -92,6 +93,10 @@ ETP_DEVICE float dot8(const uint4& a, const uint4& c) {
   }
   return s;
 }
+
+// batch row of the K / V tensor that query batch b reads (kept out of line: inlined, its load lengthens live ranges
+// in the control loop enough to add spills)
+__device__ __noinline__ int kv_row_of(const int32_t* kv_rows, int b) { return __ldg(kv_rows + b); }
 
 template <bool kPair>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -160,9 +165,10 @@ attention_bwd_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
       };
       auto load_kv = [&](int item, int j, int st) {
         const int b = item / p.heads, h = item % p.heads;
+        const int kvb = p.kv_rows ? kv_row_of(p.kv_rows, b) : b;
         mbar_arrive_expect_tx(&kv_full[st], 2 * kTile);
-        tma_load_3d(sK + st * kTile, &tmK, &kv_full[st], h * kD, j * kBK, b);
-        tma_load_3d(sV + st * kTile, &tmV, &kv_full[st], h * kD, j * kBK, b);
+        tma_load_3d(sK + st * kTile, &tmK, &kv_full[st], h * kD, j * kBK, kvb);
+        tma_load_3d(sV + st * kTile, &tmV, &kv_full[st], h * kD, j * kBK, kvb);
       };
       const int dbg_base = 0;
       ETP_DBG(0);
@@ -486,9 +492,11 @@ int attention_bwd_tc(const AttnBwdArgs& a, cudaStream_t stream) {
   if (rc) return rc;
   rc = get_tmap_3d(a.dout, W, a.Sq, a.B, a.lddo, static_cast<uint64_t>(a.Sq) * a.lddo, kD, kBQ, &tdo);
   if (rc) return rc;
-  rc = get_tmap_3d(a.k, W, a.Sk, a.B, a.ldk, static_cast<uint64_t>(a.Sk) * a.ldk, kD, kBK, &tk);
+  const int kvB = a.kv_rows ? a.kv_B : a.B;
+  ETP_REQUIRE(kvB > 0, "attention_bwd_tc: kv_B must be given with kv_rows");
+  rc = get_tmap_3d(a.k, W, a.Sk, kvB, a.ldk, static_cast<uint64_t>(a.Sk) * a.ldk, kD, kBK, &tk);
   if (rc) return rc;
-  rc = get_tmap_3d(a.v, W, a.Sk, a.B, a.ldv, static_cast<uint64_t>(a.Sk) * a.ldv, kD, kBK, &tv);
+  rc = get_tmap_3d(a.v, W, a.Sk, kvB, a.ldv, static_cast<uint64_t>(a.Sk) * a.ldv, kD, kBK, &tv);
   if (rc) return rc;
   CUtensorMap tdq, tdk, tdv;
   rc = get_tmap_3d(a.dq, W, a.Sq, a.B, a.lddq, static_cast<uint64_t>(a.Sq) * a.lddq, kD, kBQ, &tdq);
@@ -510,6 +518,7 @@ int attention_bwd_tc(const AttnBwdArgs& a, cudaStream_t stream) {
   d.dq = a.dq; d.dk = a.dk; d.dv = a.dv; d.lddq = a.lddq; d.lddk = a.lddk; d.lddv = a.lddv;
   d.dpair_w = a.dpair_w; d.dpair_b = a.dpair_b;
   d.drop = Drop{a.drop_key, a.drop_thr, a.drop_scale};
+  d.kv_rows = a.kv_rows;
   d.dbg = g_attn_bwd_dbg;
   const int items = a.B * a.heads;
   const int grid = items < num_sms() ? items : num_sms();

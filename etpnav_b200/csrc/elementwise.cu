@@ -410,6 +410,42 @@ int add_f32(float* dst, const float* src, int64_t n, cudaStream_t stream) {
   return ETP_OK;
 }
 
+// One thread per 8 columns of a row: a 16-byte bf16 load, two 16-byte fp32 read-modify-writes.  HBM-bound.
+__global__ void kv_grad_accumulate_kernel(const bf16* __restrict__ dkv, const int32_t* __restrict__ rows, int L,
+                                          int w8, int64_t n8, float* __restrict__ acc) {
+  griddep_launch();  // PDL (common.cuh): let the next kernel get scheduled ...
+  griddep_wait();    // ... and wait for the previous one before touching memory
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n8;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t r = i / w8;
+    const int c = static_cast<int>(i - r * w8);
+    const int b = static_cast<int>(r / L), l = static_cast<int>(r - static_cast<int64_t>(b) * L);
+    const int64_t dst = (static_cast<int64_t>(rows ? __ldg(rows + b) : b) * L + l) * w8 + c;
+    const uint4 g = __ldg(reinterpret_cast<const uint4*>(dkv) + i);
+    float4* a = reinterpret_cast<float4*>(acc) + 2 * dst;
+    float4 a0 = a[0], a1 = a[1];
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&g);
+    float2 f;
+    f = __bfloat1622float2(h[0]); a0.x += f.x; a0.y += f.y;
+    f = __bfloat1622float2(h[1]); a0.z += f.x; a0.w += f.y;
+    f = __bfloat1622float2(h[2]); a1.x += f.x; a1.y += f.y;
+    f = __bfloat1622float2(h[3]); a1.z += f.x; a1.w += f.y;
+    a[0] = a0; a[1] = a1;
+  }
+}
+int kv_grad_accumulate(const bf16* dkv, const int32_t* rows, int B, int L, int width, float* acc, cudaStream_t stream) {
+  ETP_REQUIRE(B > 0 && L > 0 && width > 0 && width % 8 == 0, "kv_grad_accumulate: bad shape");
+  ETP_REQUIRE((reinterpret_cast<uintptr_t>(dkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(acc) & 15) == 0,
+              "kv_grad_accumulate: alignment");
+  const int64_t n8 = static_cast<int64_t>(B) * L * (width / 8);
+  int64_t blocks = (n8 + 255) / 256;
+  if (blocks > 8 * num_sms()) blocks = 8 * num_sms();
+  ETP_CHECK_CUDA(launch_pdl(kv_grad_accumulate_kernel, dim3(static_cast<int>(blocks)), dim3(256), 0, stream, dkv, rows, L,
+                            width / 8, n8, acc));
+  ETP_LAUNCHED();
+  return ETP_OK;
+}
+
 // keep flags of elements [0, n) of one dropout site, exactly as the fused kernels evaluate them (test utility)
 __global__ void dropout_mask_kernel(const Drop d, int64_t n, uint8_t* __restrict__ out) {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;

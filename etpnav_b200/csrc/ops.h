@@ -71,6 +71,9 @@ int colsum_bf16_grouped(const ColsumJob* jobs, int n, cudaStream_t stream);
 int cast_f32_to_bf16(const float* x, bf16* y, int64_t n, cudaStream_t stream);
 int dropout_mask(DropHost d, int64_t n, uint8_t* out, cudaStream_t stream);  // keep flags of one site (tests)
 int add_f32(float* dst, const float* src, int64_t n, cudaStream_t stream);  // dst += src
+// acc[rows[b]*L + l, :] += dkv[b*L + l, :] over b < B, l < L (fp32 += bf16; rows == nullptr: identity; width % 8 == 0).
+// The rows of one call must be distinct: there are no atomics.
+int kv_grad_accumulate(const bf16* dkv, const int32_t* rows, int B, int L, int width, float* acc, cudaStream_t stream);
 
 // ---- token packing (pack.cu) ----------------------------------------------------------------------
 struct PanoPackArgs {
@@ -146,7 +149,7 @@ struct AttnArgs {
   uint32_t drop_key = 0, drop_thr = 0;
   float drop_scale = 1.0f;
   // optional: K / V live in a tensor of kv_B batch rows and query batch b reads row kv_rows[b] of it (device int32 [B]);
-  // the episode-level text K|V cache of an inference rollout whose batch shrinks (etp_nav_inputs.txt_kv_rows)
+  // the episode-level text K|V cache of a rollout whose batch shrinks (etp_nav_inputs.txt_kv_rows)
   const int32_t* kv_rows = nullptr;
   int kv_B = 0;
 };
@@ -175,6 +178,10 @@ struct AttnBwdArgs {
   float* dpair_b = nullptr;  // += sum dS          (sprel_linear.bias grad)
   uint32_t drop_key = 0, drop_thr = 0;  // the forward's attention-probability dropout (same key)
   float drop_scale = 1.0f;
+  // optional, as in AttnArgs: K / V are READ from row kv_rows[b] of a kv_B-row tensor; dK / dV are still written compact
+  // (batch b at row b) — the training rollout's text K|V cache, whose gradient is gathered by kv_grad_accumulate
+  const int32_t* kv_rows = nullptr;
+  int kv_B = 0;
 };
 int attention_bwd(const AttnBwdArgs& a, cudaStream_t stream);      // CUDA-core, any shape
 int attention_bwd_dispatch(const AttnBwdArgs& a, cudaStream_t stream);

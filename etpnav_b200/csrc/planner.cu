@@ -36,10 +36,12 @@ void LayerRecord::carve(Arena& ar, int rows, int kv_rows, int B, int Sq, bool cr
   xb = ar.take<bf16>(r * kH);
 }
 
-void NavRecord::carve(Arena& ar, int B, int N, int L, int X, bool training) {
+void NavRecord::carve(Arena& ar, int B, int N, int L, int X, bool training, bool txt_cached) {
   const size_t rows = static_cast<size_t>(B) * N;
-  txtb = ar.take<bf16>(static_cast<size_t>(B) * L * kH);
-  kv_all = ar.take<bf16>(static_cast<size_t>(B) * L * 2 * kH * (X > 0 ? X : 1));
+  if (!txt_cached) {
+    txtb = ar.take<bf16>(static_cast<size_t>(B) * L * kH);
+    kv_all = ar.take<bf16>(static_cast<size_t>(B) * L * 2 * kH * (X > 0 ? X : 1));
+  }
   x0b = ar.take<bf16>(rows * kH);
   pos_lin = ar.take<float>(rows * kH);
   pos_stats = ar.take<float>(rows * 2);
@@ -53,7 +55,7 @@ void NavRecord::carve(Arena& ar, int B, int N, int L, int X, bool training) {
   for (int i = 0; i < X; ++i) {
     if (!training) ar.off = mark;  // inference: all layers alias one scratch record
     layers[i].carve(ar, static_cast<int>(rows), 0, B, N, true);
-    layers[i].kv = kv_all + static_cast<size_t>(i) * 2 * kH;  // slice of the all-layer K|V buffer
+    if (kv_all) layers[i].kv = kv_all + static_cast<size_t>(i) * 2 * kH;  // slice of the all-layer K|V buffer
     layers[i].ldkv = X * 2 * kH;
   }
 }
@@ -184,19 +186,21 @@ int forward_navigation(const etp_nav_weights& w, const etp_nav_inputs& in, float
   const int B = in.B, N = in.N, L = in.L, X = w.num_x_layers;
   ETP_REQUIRE(B > 0 && N > 0 && L > 0 && X >= 0, "forward_navigation: bad shape");
   ETP_REQUIRE(N <= 1024 && L <= 1024, "forward_navigation: at most 1024 nodes / tokens");
+  const bf16* kv_cache = static_cast<const bf16*>(in.txt_kv_all);
+  if (kv_cache) {
+    ETP_REQUIRE(X > 0, "forward_navigation: a text K|V cache needs at least one x-layer");
+    ETP_REQUIRE(in.txt_kv_rows == nullptr || in.txt_kv_batch > 0, "forward_navigation: txt_kv_batch must be given with txt_kv_rows");
+  }
+  // with the cache the record has no text-side part: the backward reads K|V from the cache and hands dK|dV to the
+  // caller's accumulator (etp_nav_inputs.txt_kv_grad), whose one weight / data gradient runs after the rollout
   Arena ar(saved, saved_bytes);
   NavRecord rec;
-  rec.carve(ar, B, N, L, X, training);
+  rec.carve(ar, B, N, L, X, training, kv_cache != nullptr);
   ETP_REQUIRE(ar.off <= saved_bytes, "forward_navigation: saved buffer too small");
   const int rows = B * N;
   DropCtx dc;
   if (in.dropout) { dc.seed = in.dropout->seed; dc.p_hidden = in.dropout->p_hidden; dc.p_attn = in.dropout->p_attn; dc.p_head = in.dropout->p_head; }
 
-  const bf16* kv_cache = static_cast<const bf16*>(in.txt_kv_all);
-  if (kv_cache) {
-    ETP_REQUIRE(!training, "forward_navigation: the text K|V cache is an inference feature (the backward needs txt_embeds)");
-    ETP_REQUIRE(in.txt_kv_rows == nullptr || in.txt_kv_batch > 0, "forward_navigation: txt_kv_batch must be given with txt_kv_rows");
-  }
   const bf16* txtb = static_cast<const bf16*>(in.txt_embeds_bf16);
   if (txtb == nullptr && kv_cache == nullptr) {
     ETP_REQUIRE(in.txt_embeds != nullptr, "forward_navigation: txt_embeds (fp32) or txt_embeds_bf16 is required");
@@ -405,10 +409,10 @@ int forward_lang2visn(const etp_nav_weights& w, const etp_nav_inputs& in, float*
   return ETP_OK;
 }
 
-static size_t record_bytes_nav(int B, int N, int L, int X, bool training) {
+static size_t record_bytes_nav(int B, int N, int L, int X, bool training, bool txt_cached) {
   Arena ar(nullptr, ~size_t(0));
   NavRecord r;
-  r.carve(ar, B, N, L, X, training);
+  r.carve(ar, B, N, L, X, training, txt_cached);
   return ar.off;
 }
 
@@ -421,7 +425,10 @@ static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s)
 extern "C" {
 
 ETP_API size_t etp_nav_saved_bytes(int32_t B, int32_t N, int32_t L, int32_t X, int32_t training) {
-  return record_bytes_nav(B, N, L, X, training != 0);
+  return record_bytes_nav(B, N, L, X, training != 0, false);
+}
+ETP_API size_t etp_nav_kv_saved_bytes(int32_t B, int32_t N, int32_t L, int32_t X, int32_t training) {
+  return record_bytes_nav(B, N, L, X, training != 0, true);
 }
 ETP_API size_t etp_pano_saved_bytes(int32_t B, int32_t V, int32_t P, int32_t training) {
   Arena ar(nullptr, ~size_t(0));

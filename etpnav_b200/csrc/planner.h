@@ -49,14 +49,14 @@ struct LayerRecord {
 };
 
 struct NavRecord {
-  bf16* txtb = nullptr;
+  bf16* txtb = nullptr;    // (both left out when the text K|V come from an episode-level cache, etp_nav_inputs.txt_kv_all)
   bf16* kv_all = nullptr;  // text K|V of all layers, [B*L, X*1536]
   bf16* x0b = nullptr;
   float *pos_lin = nullptr, *pos_stats = nullptr;
   float *xa = nullptr, *xc = nullptr, *xf = nullptr;  // fp32 residual-stream scratch
   float *relu = nullptr, *sap_stats = nullptr;
   std::vector<LayerRecord> layers;
-  void carve(Arena& ar, int B, int N, int L, int X, bool training);
+  void carve(Arena& ar, int B, int N, int L, int X, bool training, bool txt_cached);
 };
 
 // forward_lang2visn (pre-training twin, forward_mlm): the instruction tokens are the query stream, the packed map

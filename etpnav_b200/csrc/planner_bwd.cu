@@ -203,9 +203,20 @@ int backward_navigation(const etp_nav_weights& w, const etp_nav_weights& g, cons
                         size_t work_bytes, float* d_txt_embeds, float* d_gmap_img_fts, cudaStream_t s) {
   const int B = in.B, N = in.N, L = in.L, X = w.num_x_layers;
   const int rows = B * N, kv_rows = B * L;
+  // episode-level text K|V cache (training rollout): K / V are read from the cache through the row map, and dK|dV of all
+  // layers are added into the caller's accumulator instead of becoming this step's text-side weight / data gradients
+  const bf16* kv_cache = static_cast<const bf16*>(in.txt_kv_all);
+  float* kv_grad = in.txt_kv_grad;
+  if (kv_cache || kv_grad) {
+    ETP_REQUIRE(kv_cache && kv_grad, "backward_navigation: txt_kv_all and txt_kv_grad go together (the record of a cached "
+                                     "forward has no text side)");
+    ETP_REQUIRE(X > 0, "backward_navigation: a text K|V cache needs at least one x-layer");
+    ETP_REQUIRE(d_txt_embeds == nullptr, "backward_navigation: with txt_kv_grad, d_txt_embeds comes from etp_backward_text_kv");
+    ETP_REQUIRE(in.txt_kv_rows == nullptr || in.txt_kv_batch > 0, "backward_navigation: txt_kv_batch must be given with txt_kv_rows");
+  }
   Arena ar(saved, saved_bytes);
   NavRecord rec;
-  rec.carve(ar, B, N, L, X, true);
+  rec.carve(ar, B, N, L, X, true, kv_cache != nullptr);
   ETP_REQUIRE(ar.off <= saved_bytes, "backward_navigation: saved buffer too small");
   Arena wa(work, work_bytes);
   BwdScratch sc;
@@ -250,6 +261,11 @@ int backward_navigation(const etp_nav_weights& w, const etp_nav_weights& g, cons
     AttnBwdArgs at;
     at.B = B; at.heads = kHeads; at.Sq = N; at.Sk = L;
     at.q = r.q; at.ldq = kH; at.k = r.kv; at.ldk = r.ldkv; at.v = r.kv + kH; at.ldv = r.ldkv;
+    if (kv_cache) {  // as in the forward: layer i's slice of the cached rows, read through the batch-row map
+      at.k = kv_cache + static_cast<size_t>(i) * 2 * kH; at.v = at.k + kH;
+      at.ldk = at.ldv = ldkv;
+      at.kv_rows = in.txt_kv_rows; at.kv_B = in.txt_kv_rows ? in.txt_kv_batch : B;
+    }
     at.out = r.ctx1; at.ldo = kH; at.dout = sc.dctx; at.lddo = kH; at.lse = r.lse1; at.dvec = sc.dvec;
     at.scale = 0.125f; at.key_valid = in.txt_masks; at.mask_value = -10000.0f;
     bf16* dkv_i = sc.dkv + static_cast<size_t>(i) * 2 * kH;  // this layer's slice of [B*L, X*1536]
@@ -277,7 +293,9 @@ int backward_navigation(const etp_nav_weights& w, const etp_nav_weights& g, cons
   if (in.img_grad_event) ETP_CHECK_CUDA(cudaEventRecord(static_cast<cudaEvent_t>(in.img_grad_event), s));
   // text side, all layers at once: kv_all = txt . Wkv_all^T + b  ->  one wgrad, one dgrad (bias grads: above); they leave
   // side_sm_reserve SMs to the stream that now runs the panorama backward
-  if (X > 0) {
+  if (kv_grad) {
+    ETP_TRY(kv_grad_accumulate(sc.dkv, in.txt_kv_rows, B, L, ldkv, kv_grad, s));
+  } else if (X > 0) {
     const bf16* txtb = in.txt_embeds_bf16 ? static_cast<const bf16*>(in.txt_embeds_bf16) : rec.txtb;
     const int prev = get_sm_reserve();
     if (in.side_sm_reserve > 0) set_sm_reserve(prev + in.side_sm_reserve);
@@ -487,6 +505,31 @@ int backward_txt(const etp_txt_weights& w, const etp_txt_weights& g, const int64
   return ETP_OK;
 }
 
+// Backward of etp_encode_text_kv for a training rollout: the accumulated dK|dV of every step, cast to bf16 once, make ONE
+// weight gradient of the stacked key|value projection and (optionally) ONE data gradient of txt_embeds.  (The value-bias
+// gradients were taken step by step by backward_navigation; the key-bias gradient is zero.)
+int backward_text_kv(const etp_nav_weights& w, const etp_nav_weights& g, const float* txt_embeds, const bf16* txt_embeds_bf16,
+                     int B, int L, const float* dkv_acc, float* d_txt_embeds, void* work, cudaStream_t s) {
+  const int X = w.num_x_layers;
+  ETP_REQUIRE(B > 0 && L > 0 && X > 0, "backward_text_kv: bad shape");
+  const size_t rows = static_cast<size_t>(B) * L, ldkv = static_cast<size_t>(X) * 2 * kH;
+  Arena wa(work, ~size_t(0));
+  bf16* dkvb = wa.take<bf16>(rows * ldkv);
+  const bf16* txtb = txt_embeds_bf16;
+  if (txtb == nullptr) {
+    bf16* t = wa.take<bf16>(rows * kH);
+    ETP_TRY(cast_f32_to_bf16(txt_embeds, t, static_cast<int64_t>(rows) * kH, s));
+    txtb = t;
+  }
+  ETP_TRY(cast_f32_to_bf16(dkv_acc, dkvb, static_cast<int64_t>(rows * ldkv), s));
+  ETP_TRY(wgrad(dkvb, static_cast<int>(rows), static_cast<int>(ldkv), static_cast<int>(ldkv), txtb, kH, kH,
+                const_cast<void*>(g.xkv_all_w), s));
+  if (d_txt_embeds)
+    ETP_TRY(dgrad(dkvb, static_cast<int>(rows), static_cast<int>(ldkv), static_cast<int>(ldkv), w.xkv_all_w, kH, nullptr,
+                  d_txt_embeds, nullptr, 0, nullptr, s));
+  return ETP_OK;
+}
+
 static size_t work_bytes_for(size_t rows, size_t kv_rows, size_t bhs, size_t kv_layers = 1) {
   Arena wa(nullptr, ~size_t(0));
   BwdScratch sc;
@@ -507,6 +550,13 @@ extern "C" {
 ETP_API size_t etp_nav_bwd_work_bytes(int32_t B, int32_t N, int32_t L, int32_t num_x_layers) {
   return work_bytes_for(static_cast<size_t>(B) * N, static_cast<size_t>(B) * L, static_cast<size_t>(B) * kHeads * (N > L ? N : L),
                         num_x_layers > 0 ? num_x_layers : 1);
+}
+ETP_API size_t etp_text_kv_bwd_work_bytes(int32_t B, int32_t L, int32_t num_x_layers) {
+  Arena wa(nullptr, ~size_t(0));
+  const size_t rows = static_cast<size_t>(B) * L;
+  wa.take<bf16>(rows * 2 * kH * (num_x_layers > 0 ? num_x_layers : 1));
+  wa.take<bf16>(rows * kH);
+  return wa.off;
 }
 ETP_API size_t etp_pano_bwd_work_bytes(int32_t B, int32_t V) {
   return work_bytes_for(static_cast<size_t>(B) * V, 0, static_cast<size_t>(B) * kHeads * V);
@@ -534,6 +584,13 @@ ETP_API int etp_backward_navigation(const etp_nav_weights* w, const etp_nav_weig
   ETP_REQUIRE(w && grads && in && saved && work, "etp_backward_navigation: null argument");
   return backward_navigation(*w, *grads, *in, d_gmap_embeds, d_global_logits, saved, saved_bytes, work, work_bytes,
                              d_txt_embeds, d_gmap_img_fts, S(stream));
+}
+ETP_API int etp_backward_text_kv(const etp_nav_weights* w, const etp_nav_weights* grads, const float* txt_embeds,
+                                 const void* txt_embeds_bf16, int32_t B, int32_t L, const float* dkv_acc, float* d_txt_embeds,
+                                 void* work, void* stream) {
+  ETP_REQUIRE(w && grads && dkv_acc && work && (txt_embeds || txt_embeds_bf16), "etp_backward_text_kv: null argument");
+  return backward_text_kv(*w, *grads, txt_embeds, static_cast<const bf16*>(txt_embeds_bf16), B, L, dkv_acc, d_txt_embeds,
+                          work, S(stream));
 }
 ETP_API int etp_backward_panorama(const etp_pano_weights* w, const etp_pano_weights* grads, const etp_pano_inputs* in,
                                   const uint8_t* pano_masks, const float* d_pano_embeds, void* saved, size_t saved_bytes,

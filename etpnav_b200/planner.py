@@ -51,7 +51,7 @@ class NavInputs(C.Structure):
                               "gmap_masks", "gmap_visited_masks", "gmap_pair_dists")] + [
         ("dropout", C.POINTER(Dropout)), ("layer_done_events", C.POINTER(p_void)), ("txt_embeds_bf16", p_void),
         ("txt_kv_all", p_void), ("txt_kv_rows", p_void), ("txt_kv_batch", i32),
-        ("side_sm_reserve", i32), ("img_ready_event", p_void), ("img_grad_event", p_void)]
+        ("side_sm_reserve", i32), ("img_ready_event", p_void), ("img_grad_event", p_void), ("txt_kv_grad", p_void)]
 
 
 class PanoLayerWeights(C.Structure):
@@ -85,6 +85,12 @@ def _declare():
     L = _L.lib()
     L.etp_nav_saved_bytes.restype = C.c_size_t
     L.etp_nav_saved_bytes.argtypes = [i32] * 5
+    L.etp_nav_kv_saved_bytes.restype = C.c_size_t
+    L.etp_nav_kv_saved_bytes.argtypes = [i32] * 5
+    L.etp_text_kv_bwd_work_bytes.restype = C.c_size_t
+    L.etp_text_kv_bwd_work_bytes.argtypes = [i32] * 3
+    L.etp_backward_text_kv.argtypes = [C.POINTER(NavWeights), C.POINTER(NavWeights), p_void, p_void, i32, i32, p_void, p_void,
+                                       p_void, p_void]
     L.etp_pano_saved_bytes.restype = C.c_size_t
     L.etp_pano_saved_bytes.argtypes = [i32] * 4
     L.etp_txt_saved_bytes.restype = C.c_size_t
@@ -123,16 +129,30 @@ def _declare():
     _declared = True
 
 
+class _TextKVGrad:
+    """Gradient side of a training ``TextKV`` handle, shared by every indexed copy of it: the rollout's fp32 dK|dV
+    accumulator ``[B0 * L, X * 1536]`` and whether its backward has run.  (It holds no autograd tensor, so the backward
+    node that owns it forms no reference cycle.)"""
+
+    def __init__(self, acc):
+        self.acc, self.done = acc, False
+
+
 class TextKV:
     """Episode-level handle of the instruction's key|value projections for ALL cross-modal layers
     (``B200Planner.encode_text_kv``): bf16 ``[B0 * L, X * 1536]``, computed ONCE per episode instead of at every step
     of every layer (the reference recomputes them although ``txt_embeds`` is constant over the episode,
-    vilmodel_cmt.py:326-328).  Pass it to ``forward_navigation`` in place of ``txt_embeds`` (inference / eval rollouts).
+    vilmodel_cmt.py:326-328).  Pass it to ``forward_navigation`` in place of ``txt_embeds``.
     Indexing it like the trainer indexes ``all_txt_embeds[not_done_index]`` (ss_trainer_ETP.py:819-821) keeps the cache
-    and records the surviving episodes as a row map — no data moves."""
+    and records the surviving episodes as a row map — no data moves.
 
-    def __init__(self, kv_all, batch, length, rows=None):
+    A training handle (made with gradients wanted) also carries ``grad`` (the rollout's dK|dV accumulator) and ``token``,
+    the autograd output of the encoding: every navigation step that reads the handle hangs off it, and after the last of
+    their backwards one node turns the accumulator into the key|value weight gradient and d ``txt_embeds``."""
+
+    def __init__(self, kv_all, batch, length, rows=None, grad=None, token=None):
         self.kv_all, self.batch, self.length, self.rows = kv_all, batch, length, rows
+        self.grad, self.token = grad, token
 
     def __len__(self):
         return self.batch if self.rows is None else int(self.rows.numel())
@@ -148,7 +168,7 @@ class TextKV:
             idx = torch.as_tensor(idx, device=dev)
         idx = idx.to(dev)
         rows = base[idx] if idx.dtype == torch.bool else base[idx.long()]
-        return TextKV(self.kv_all, self.batch, self.length, rows.to(torch.int32).contiguous())
+        return TextKV(self.kv_all, self.batch, self.length, rows.to(torch.int32).contiguous(), self.grad, self.token)
 
 
 class _Holder(nn.Module):
@@ -544,11 +564,21 @@ class B200Planner(nn.Module):
         aux = (self._mask_u8(txt_masks), gmap_step_ids.contiguous().long(), _f32c(gmap_pos_fts),
                self._mask_u8(gmap_masks), self._mask_u8(gmap_visited_masks), _f32c(gmap_pair_dists))
         if isinstance(txt_embeds, TextKV):
-            if self.precision != "bf16" or self._wants_grad("nav", gmap_img_fts):
-                raise _L.EtpError("a TextKV handle serves bf16-mode inference (torch.no_grad()): the backward needs txt_embeds")
-            if len(txt_embeds) != gmap_img_fts.shape[0] or txt_embeds.length != txt_masks.shape[1]:
+            kv = txt_embeds
+            if kv.grad is not None and kv.grad.done:
+                raise _L.EtpError("this TextKV handle's backward has run: encode the instruction again for a new rollout")
+            train = kv.grad is not None and torch.is_grad_enabled()
+            if self.precision != "bf16" or (not train and self._wants_grad("nav", gmap_img_fts)):
+                raise _L.EtpError("a TextKV handle serves the bf16 mode, and only one made by encode_text_kv with gradients "
+                                  "enabled can be trained through")
+            if len(kv) != gmap_img_fts.shape[0] or kv.length != txt_masks.shape[1]:
                 raise ValueError("TextKV handle and the step's batch disagree: index the handle like all_txt_embeds")
-            embeds, logits, _, _ = _nav_forward(self, txt_embeds, _f32c(gmap_img_fts), aux, 0, None)
+            if train:
+                drop = self._next_dropout()
+                params = [] if self._direct_grad is not None else [self._pmap[n] for n in self._nav_kv_step_names()]
+                embeds, logits = _NavKVFn.apply(self, kv.token, gmap_img_fts, kv, aux, drop, self._anchor_t(), *params)
+            else:
+                embeds, logits, _, _ = _nav_forward(self, kv, _f32c(gmap_img_fts), aux, 0, None)
             return {"gmap_embeds": embeds, "global_logits": logits}
         if self.precision == "high":
             self._hp_guard(self._wants_grad("nav", txt_embeds, gmap_img_fts))
@@ -564,20 +594,36 @@ class B200Planner(nn.Module):
 
     def encode_text_kv(self, txt_embeds):
         """Once per episode (after ``forward_txt``): the key|value projections of the instruction for every x-layer, as a
-        ``TextKV`` handle that ``forward_navigation`` accepts in place of ``txt_embeds`` (eval / inference rollouts).
-        Bit-identical to what the un-cached step computes; saves the [B*L,768] x [X*1536,768] GEMM at every step."""
+        ``TextKV`` handle that ``forward_navigation`` accepts in place of ``txt_embeds``.
+        Bit-identical to what the un-cached step computes; saves the [B*L,768] x [X*1536,768] GEMM at every step.
+
+        With gradients enabled (bf16 mode, and ``txt_embeds`` or a cross-modal key/value weight requires grad) the handle
+        can be trained through over a whole rollout: each step's backward adds its dK|dV into the handle's accumulator
+        instead of running the text-side weight and data gradient GEMMs and keeping the step's K|V, and one node after the
+        rollout runs them once.  Under ``torch.no_grad()`` it is an inference handle."""
         self._refresh_cache()
-        t = _txtc(txt_embeds)
-        B, Lt = t.shape[:2]
         X = self.config.num_x_layers
         if X == 0:
             raise ValueError("no cross-modal layers: nothing to cache")
-        kv = torch.empty(B * Lt, X * 1536, dtype=torch.bfloat16, device=t.device)
-        work = torch.empty(B * Lt * 768, dtype=torch.bfloat16, device=t.device) if t.dtype != torch.bfloat16 else None
-        _L._check(_L.lib().etp_encode_text_kv(C.byref(self._structs["nav"]), _L.ptr(t) if work is not None else None,
-                                              _L.ptr(t) if work is None else None, B, Lt, _L.ptr(kv), _L.ptr(work),
-                                              _L.stream_ptr()), "etp_encode_text_kv")
-        return TextKV(kv, B, Lt)
+        if torch.is_grad_enabled() and self.precision == "bf16" and (
+                txt_embeds.requires_grad or any(self._pmap[n].requires_grad for n in self._kv_weight_names())):
+            params = [] if self._direct_grad is not None else [self._pmap[n] for n in self._kv_weight_names()]
+            box = []
+            token = _TextKVFn.apply(self, txt_embeds, box, self._anchor_t(), *params)
+            kv, grad = box
+            return TextKV(kv, txt_embeds.shape[0], txt_embeds.shape[1], grad=grad, token=token)
+        t = _txtc(txt_embeds)
+        return TextKV(_encode_text_kv(self, t), t.shape[0], t.shape[1])
+
+    def _kv_weight_names(self):
+        # key|value weights of every cross-modal layer: the stacked [X*1536, 768] operand of the text K|V GEMM
+        return [f"global_encoder.encoder.x_layers.{i}.visual_attention.att.{kv}.weight"
+                for i in range(self.config.num_x_layers) for kv in ("key", "value")]
+
+    def _nav_kv_step_names(self):
+        # the navigation group minus the key|value weights, whose gradient the training TextKV handle's node returns
+        kvw = set(self._kv_weight_names())
+        return [n for n in self._group_names("nav") if n not in kvw]
 
     # ------------------------------------------------------------------ training helper
     def make_trainer(self, lr=1e-5, world_size=1, **kw):
@@ -645,6 +691,17 @@ def _nav_inputs(txt, img, aux, drop=None):
     return ni
 
 
+def _encode_text_kv(m, t):
+    """etp_encode_text_kv of txt_embeds ``t`` (fp32 or bf16 [B,L,768]) -> bf16 [B*L, X*1536]."""
+    B, Lt = t.shape[:2]
+    kv = torch.empty(B * Lt, m.config.num_x_layers * 1536, dtype=torch.bfloat16, device=t.device)
+    work = torch.empty(B * Lt * 768, dtype=torch.bfloat16, device=t.device) if t.dtype != torch.bfloat16 else None
+    _L._check(_L.lib().etp_encode_text_kv(C.byref(m._structs["nav"]), _L.ptr(t) if work is not None else None,
+                                          _L.ptr(t) if work is None else None, B, Lt, _L.ptr(kv), _L.ptr(work),
+                                          _L.stream_ptr()), "etp_encode_text_kv")
+    return kv
+
+
 def _nav_forward(m, txt, img, aux, training, drop=None, img_ready_event=None, side_sm_reserve=0):
     B, N = img.shape[:2]
     Lt = txt.shape[1]
@@ -655,7 +712,8 @@ def _nav_forward(m, txt, img, aux, training, drop=None, img_ready_event=None, si
     ni.side_sm_reserve = side_sm_reserve
     embeds = torch.empty(B, N, 768, device=img.device, dtype=torch.float32)
     logits = torch.empty(B, N, device=img.device, dtype=torch.float32)
-    nbytes = L.etp_nav_saved_bytes(B, N, Lt, m.config.num_x_layers, training)
+    saved_bytes = L.etp_nav_kv_saved_bytes if isinstance(txt, TextKV) else L.etp_nav_saved_bytes
+    nbytes = saved_bytes(B, N, Lt, m.config.num_x_layers, training)
     saved = torch.empty(nbytes, dtype=torch.uint8, device=img.device)
     _L._check(L.etp_forward_navigation(C.byref(m._structs["nav"]), C.byref(ni), _L.ptr(embeds), _L.ptr(logits),
                                        _L.ptr(saved), nbytes, training, _L.stream_ptr()), "etp_forward_navigation")
@@ -714,7 +772,9 @@ def _nav_backward_raw(m, txt, img, aux, drop, saved, de, dl, want_dtxt, want_dim
     if img_grad_event is not None:
         ni.img_grad_event = C.c_void_p(img_grad_event)
     ni.side_sm_reserve = side_sm_reserve
-    d_txt = torch.empty(txt.shape, dtype=torch.float32, device=txt.device) if want_dtxt else None
+    if isinstance(txt, TextKV):
+        ni.txt_kv_grad = _L.ptr(txt.grad.acc)
+    d_txt = torch.empty(txt.shape, dtype=torch.float32, device=img.device) if want_dtxt else None
     d_img = (d_img_out if d_img_out is not None else torch.empty_like(img)) if want_dimg else None
     wbytes = L.etp_nav_bwd_work_bytes(B, N, Lt, m.config.num_x_layers)
     work = torch.empty(wbytes, dtype=torch.uint8, device=img.device)
@@ -790,6 +850,75 @@ class _NavFn(torch.autograd.Function):
         if d_img is not None and d_img.dtype != ctx.in_dtypes[1]:
             d_img = d_img.to(ctx.in_dtypes[1])
         return (None, d_txt, d_img, None, None, None, *pg)
+
+
+class _TextKVFn(torch.autograd.Function):
+    """encode_text_kv of a training rollout.  Output: a token the navigation steps that read the handle take as input, so
+    that this node's backward runs after all of theirs; it turns the accumulated dK|dV into the key|value weight gradient
+    and d txt_embeds (one GEMM each)."""
+
+    @staticmethod
+    def forward(ctx, m, txt_embeds, box, anchor, *params):
+        t = _txtc(txt_embeds)
+        kv = _encode_text_kv(m, t)
+        grad = _TextKVGrad(torch.zeros(kv.shape, dtype=torch.float32, device=kv.device))
+        box.extend((kv, grad))
+        ctx.m, ctx.t, ctx.grad, ctx.nparams, ctx.in_dtype = m, t, grad, len(params), txt_embeds.dtype
+        return torch.zeros(1, device=kv.device)
+
+    @staticmethod
+    def backward(ctx, _d_token):
+        m, t, grad = ctx.m, ctx.t, ctx.grad
+        if grad.done:
+            raise _L.EtpError("the TextKV handle's backward already ran (retain_graph is not supported through it)")
+        L = _L.lib()
+        B, Lt = t.shape[:2]
+        gbuf, gstart, per_call = m._grad_target("nav")
+        gst = m._grad_structs_for(gbuf, gstart)
+        d_txt = torch.empty(t.shape, dtype=torch.float32, device=t.device) if ctx.needs_input_grad[1] else None
+        work = torch.empty(L.etp_text_kv_bwd_work_bytes(B, Lt, m.config.num_x_layers), dtype=torch.uint8, device=t.device)
+        bf = t.dtype == torch.bfloat16
+        _L._check(L.etp_backward_text_kv(C.byref(m._structs["nav"]), C.byref(gst["nav"]), None if bf else _L.ptr(t),
+                                         _L.ptr(t) if bf else None, B, Lt, _L.ptr(grad.acc), _L.ptr(d_txt), _L.ptr(work),
+                                         _L.stream_ptr()), "etp_backward_text_kv")
+        grad.done, grad.acc = True, None
+        pg = _param_grads(m, m._kv_weight_names(), gbuf, gstart, per_call, ctx.nparams)
+        if d_txt is not None and d_txt.dtype != ctx.in_dtype:
+            d_txt = d_txt.to(ctx.in_dtype)
+        return (None, d_txt, None, None, *pg)
+
+
+class _NavKVFn(torch.autograd.Function):
+    """forward_navigation through a training TextKV handle: the record leaves out the step's K|V and bf16 txt_embeds, and
+    the backward adds dK|dV into the handle's accumulator (the token's gradient is zero)."""
+
+    @staticmethod
+    def forward(ctx, m, token, gmap_img_fts, kv, aux, drop, anchor, *params):
+        img = _f32c(gmap_img_fts)
+        embeds, logits, saved, _ = _nav_forward(m, kv, img, aux, 1, drop)
+        # the handle minus its token: the token's node must not be kept alive from here
+        ctx.kv = TextKV(kv.kv_all, kv.batch, kv.length, kv.rows, kv.grad)
+        ctx.m, ctx.saved, ctx.keep, ctx.nparams, ctx.drop = m, saved, (img, aux), len(params), drop
+        ctx.in_dtype = gmap_img_fts.dtype
+        return embeds, logits
+
+    @staticmethod
+    def backward(ctx, d_embeds, d_logits):
+        m, kv = ctx.m, ctx.kv
+        img, aux = ctx.keep
+        if kv.grad.done:
+            raise _L.EtpError("the TextKV handle's backward already ran (retain_graph is not supported through it)")
+        de = _f32c(d_embeds) if d_embeds is not None else None
+        dl = _f32c(d_logits) if d_logits is not None else None
+        if dl is not None:
+            dl = torch.nan_to_num(dl, nan=0.0, posinf=0.0, neginf=0.0)
+        _, d_img, gbuf, gstart, per_call = _nav_backward_raw(m, kv, img, aux, ctx.drop, ctx.saved, de, dl, False,
+                                                             ctx.needs_input_grad[2])
+        pg = _param_grads(m, m._nav_kv_step_names(), gbuf, gstart, per_call, ctx.nparams)
+        if d_img is not None and d_img.dtype != ctx.in_dtype:
+            d_img = d_img.to(ctx.in_dtype)
+        d_token = torch.zeros(1, device=img.device) if ctx.needs_input_grad[1] else None
+        return (None, d_token, d_img, None, None, None, None, *pg)
 
 
 class _PanoFn(torch.autograd.Function):

@@ -261,12 +261,13 @@ typedef struct {
    * read the instruction through it (their first act on txt_embeds is a cast to bf16 for TMA anyway) and txt_embeds may be
    * NULL: a host that keeps, or stages across PCIe, the instruction embeddings in bf16 saves the cast and half the bytes. */
   const void* txt_embeds_bf16;
-  /* optional, inference only: the instruction's key|value projections of ALL x-layers, computed once per episode by
+  /* optional: the instruction's key|value projections of ALL x-layers, computed once per episode by
    * etp_encode_text_kv (bf16 [txt_kv_batch * L, num_x_layers * 1536]).  The reference recomputes them at every step of
    * every layer although txt_embeds is constant over the episode (vilmodel_cmt.py:326-328; 24 % of the forward FLOPs at
    * B64/N80/L200).  txt_kv_rows (device int32 [B], or NULL = identity) maps the step's batch rows to rows of the
    * episode batch the cache was built for: the trainer shrinks the batch as episodes finish
-   * (all_txt_embeds[not_done_index], ss_trainer_ETP.py:819-821).  With txt_kv_all set, txt_embeds may be NULL. */
+   * (all_txt_embeds[not_done_index], ss_trainer_ETP.py:819-821).  With txt_kv_all set, txt_embeds may be NULL.
+   * In training the record then has no text side (etp_nav_kv_saved_bytes) and the backward needs txt_kv_grad. */
   const void* txt_kv_all;
   const int32_t* txt_kv_rows;
   int32_t txt_kv_batch;
@@ -282,20 +283,38 @@ typedef struct {
   int32_t side_sm_reserve;
   void* img_ready_event;
   void* img_grad_event;
+  /* backward only, required with txt_kv_all (training rollout through the text K|V cache): fp32 accumulator
+   * [txt_kv_batch * L, num_x_layers * 1536] of the rollout's dK|dV.  The backward adds this step's dK|dV into row
+   * txt_kv_rows[b] * L + l (no text-side weight / data gradient GEMM runs; d_txt_embeds must be NULL); the per-layer
+   * value-bias gradients are still taken here.  After the last step, etp_backward_text_kv turns the accumulator into the
+   * key|value weight gradient and d txt_embeds.  Steps must run in order on one stream (plain read-add-write). */
+  float* txt_kv_grad;
 } etp_nav_inputs;
 
 /* Bytes of the activation record forward_navigation writes (and backward reads) when training != 0;
  * with training == 0 the size of the scratch the forward needs. */
 size_t etp_nav_saved_bytes(int32_t B, int32_t N, int32_t L, int32_t num_x_layers, int32_t training);
+/* The same with etp_nav_inputs.txt_kv_all set: no bf16 txt_embeds and no K|V of the step in the record, i.e.
+ * B*L*(num_x_layers*1536 + 768)*2 bytes less than etp_nav_saved_bytes. */
+size_t etp_nav_kv_saved_bytes(int32_t B, int32_t N, int32_t L, int32_t num_x_layers, int32_t training);
 /* GlocalTextPathNavCMT.forward_navigation (vilmodel_cmt.py:721-750).
  * outputs: gmap_embeds fp32 [B,N,768], global_logits fp32 [B,N] (-inf at visited / padded nodes). */
 int etp_forward_navigation(const etp_nav_weights* w, const etp_nav_inputs* in, float* gmap_embeds,
                            float* global_logits, void* saved, size_t saved_bytes, int32_t training, void* stream);
-/* Episode-level text K|V cache for inference rollouts: kv_all[b*L + l, i*1536 : (i+1)*1536] = key|value projection of
- * x-layer i of token (b, l) (visual_attention.att.{key,value}, vilmodel_cmt.py:327-328), bf16.  txt_embeds fp32 [B,L,768]
+/* Episode-level text K|V cache of a rollout (inference, or training with etp_nav_inputs.txt_kv_grad):
+ * kv_all[b*L + l, i*1536 : (i+1)*1536] = key|value projection of x-layer i of token (b, l)
+ * (visual_attention.att.{key,value}, vilmodel_cmt.py:327-328), bf16.  txt_embeds fp32 [B,L,768]
  * (or txt_embeds_bf16, the other NULL); work: B*L*768 bf16 of scratch (unused with the bf16 input). */
 int etp_encode_text_kv(const etp_nav_weights* w, const float* txt_embeds, const void* txt_embeds_bf16, int32_t B, int32_t L,
                        void* kv_all, void* work, void* stream);
+/* Backward of etp_encode_text_kv after a training rollout: dkv_acc = the etp_nav_inputs.txt_kv_grad accumulator
+ * [B*L, num_x_layers*1536] fp32.  Casts it to bf16, ACCUMULATES (+=) its weight gradient into grads->xkv_all_w (one GEMM) and,
+ * when d_txt_embeds [B,L,768] fp32 is non-NULL, overwrites it with the data gradient (one GEMM).  txt_embeds fp32 or
+ * txt_embeds_bf16 (the other NULL) are the embeddings the cache was built from; work: etp_text_kv_bwd_work_bytes. */
+size_t etp_text_kv_bwd_work_bytes(int32_t B, int32_t L, int32_t num_x_layers);
+int etp_backward_text_kv(const etp_nav_weights* w, const etp_nav_weights* grads, const float* txt_embeds,
+                         const void* txt_embeds_bf16, int32_t B, int32_t L, const float* dkv_acc, float* d_txt_embeds,
+                         void* work, void* stream);
 
 /* ImageEmbeddings + pano encoder (vilmodel_cmt.py:454-486; common/transformer.py:127-182) */
 typedef struct {
